@@ -86,6 +86,16 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+def dump_outputs(out_dir, point, infinity):
+    """What one MSM step hands its caller: the affine G1 result (b200zk.h layout, x then y, each four little-endian u64
+    Montgomery limbs) as sixteen 32-bit words in float64, which holds them exactly, and the infinity flag."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    words = np.ascontiguousarray(point, dtype="<u8").view("<u4").reshape(2, 8)
+    np.save(os.path.join(out_dir, "msm_g1_affine_words.npy"), words.astype(np.float64))
+    np.save(os.path.join(out_dir, "msm_g1_infinity.npy"), np.array([float(infinity)]))
+
+
 def run_reference(args):
     """CPU arm: the arkworks-equivalent restatement on the host cores, rank 0 only."""
     if int(os.environ.get("RANK", "0")) != 0:
@@ -101,8 +111,10 @@ def run_reference(args):
         cref.msm_g1(bases, scalars, cores)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        cref.msm_g1(bases, scalars, cores)
+        res = cref.msm_g1(bases, scalars, cores)
     dt = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *res)
     val = n / dt / 1e6
     sample = "full 2^%d-pair G1 MSM per step, %d OpenMP threads (windows in parallel, as arkworks+rayon)" % (LOG_N, cores)
     emit({
@@ -522,7 +534,12 @@ def main():
     ap.add_argument("--no-prove", action="store_true", help="skip the secondary Groth16-prove measurements")
     ap.add_argument("--no-multi", action="store_true", help="N > 1: skip the four-step NTT / sharded prove / strong-scaling sections")
     ap.add_argument("--no-sizes", action="store_true", help="N = 1: skip the 2^22..2^26 MSM size sweep")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last timed step's result to DIR/*.npy (float64; inputs are seeded, "
+                         "so runs with the same arguments can be compared output for output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -611,6 +628,8 @@ def main():
     t_wall = time.perf_counter() - t_wall0
     launches = net.launch_count() - l0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *(res if world == 1 else host_result()))
     ms_step = sum(times) / len(times)
     ms_step_sorted = sorted(times)
 

@@ -1,6 +1,6 @@
-"""Regenerates tests/golden/* from the reference's own fixtures under /root/reference (run in the build
-container only; the GPU box has no /root/reference).  Everything copied here is test DATA (goldens the
-reference's tests hold), never source:
+"""Regenerates tests/golden/* from the reference's own fixtures: `python tests/golden/make_golden.py <checkout of
+zkHubHQ/distributed-groth16>`.  The tests read only what this writes, never the checkout.  Everything copied here is
+test DATA (goldens the reference's tests hold), never source:
 
   sha256_proof.bin            zk-cli/test-circuits/sha256/proof.bin  (128 B, the only full-prover golden)
   reference_goldens.json      - decimal coordinates of that proof as printed in zk-cli/README.md:82
@@ -14,8 +14,14 @@ reference's tests hold), never source:
                               (public output == the KAT of groth16/examples/sha256.rs:231-233; all 30 134 constraints hold)
   complex_circuit_proof.json  the oracle's proof for witness a = 3 on that key (r = s = 0 and r, s != 0),
                               both verified against the zkey's own vk with the oracle pairing
+  reference_fixtures.npz      what tests/test_formats.py needs beside the files above to rebuild four fixture files
+                              byte for byte (SHA-256 of each original): the complex-circuit zkey (section order and
+                              section 10), its r1cs (xz-compressed), fixtures/sha256/sha256.r1cs (header, section
+                              order, wire label steps) and fixtures/million/witness.wtns (1, 999992, 1, 2, ..., 999991)
 """
+import hashlib
 import json
+import lzma
 import os
 import re
 import sys
@@ -26,7 +32,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "..", ".."))
 from oracle import bn254 as o, layout  # noqa: E402
 
-REF = "/root/reference"
+REF = None         # the reference checkout, from the command line
 
 
 def make_sha256_fixture(g):
@@ -113,8 +119,34 @@ def main():
     out["public_input"] = str(z[1])
     json.dump(out, open(os.path.join(HERE, "complex_circuit_proof.json"), "w"), indent=1)
     make_sha256_fixture(g)
+    make_fixture_rebuild_data()
     print("golden files written")
 
 
+def make_fixture_rebuild_data():
+    sha = lambda b: np.array(hashlib.sha256(b).hexdigest())
+    order = lambda secs: np.array(sorted(secs, key=lambda sid: secs[sid][0][0]), dtype=np.uint32)
+    zk = open(REF + "/ark-circom/test-vectors/complex-circuit/complex-circuit-10000-10000.zkey", "rb").read()
+    zs = o._sections(zk, b"zkey")
+    (o10, l10), = zs[10]
+    cr = open(REF + "/ark-circom/test-vectors/complex-circuit/complex-circuit-10000-10000.r1cs", "rb").read()
+    sr = open(REF + "/fixtures/sha256/sha256.r1cs", "rb").read()
+    ss = o._sections(sr, b"r1cs")
+    (o1, l1), = ss[1]
+    (o3, l3), = ss[3]
+    labels = np.frombuffer(sr, dtype="<u8", count=l3 // 8, offset=o3)
+    wtns = open(REF + "/fixtures/million/witness.wtns", "rb").read()
+    np.savez_compressed(
+        os.path.join(HERE, "reference_fixtures.npz"),
+        complex_zkey_sha256=sha(zk), complex_zkey_section_order=order(zs),
+        complex_zkey_section10=np.frombuffer(zk, dtype=np.uint8, count=l10, offset=o10),
+        complex_r1cs_sha256=sha(cr), complex_r1cs_xz=np.frombuffer(lzma.compress(cr, preset=9 | lzma.PRESET_EXTREME), dtype=np.uint8),
+        sha256_r1cs_sha256=sha(sr), sha256_r1cs_section_order=order(ss),
+        sha256_r1cs_header=np.frombuffer(sr, dtype=np.uint8, count=l1, offset=o1),
+        sha256_r1cs_label_steps=np.diff(labels, prepend=0).astype(np.uint32),
+        million_wtns_sha256=sha(wtns))
+
+
 if __name__ == "__main__":
+    REF = os.path.abspath(sys.argv[1])
     main()
